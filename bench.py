@@ -4,6 +4,7 @@ roofline of the vectorised leapfrog kernel and the CPU baseline timed beside it.
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun launches N>1)
     python bench.py --impl reference --gpus N --steps K ...   # reference arm: CPU oracle twin
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one pass of the hot path over every chain of the workload: one HMC transition (L leapfrogs), one NUTS
 transition (config 3), or one complete 200-step window-adaptation warm-up (config 4).  `value` counts executed
@@ -339,6 +340,31 @@ def ncu_traffic(kernel_key):
         return None, None
 
 
+# payload cap of --dump-outputs; with the .npy headers the files stay under 64 MB
+DUMP_BYTES = 60 * 10 ** 6
+
+
+def dump_outputs(out_dir, per_chain, shared=None):
+    """--dump-outputs: writes what the timed path returned in its last step as out_dir/<name>.npy, float32.  per_chain maps
+    names to tensors with the chains on axis 0.  When they exceed DUMP_BYTES, every one of them keeps the same seeded sample
+    of chains; chain_index.npy (float64) holds the chain indices kept.  shared holds the arrays that are not per chain."""
+    import numpy as np
+    import torch
+    shared = {k: torch.as_tensor(v) for k, v in (shared or {}).items()}
+    C = next(iter(per_chain.values())).shape[0]
+    row_bytes = 8 + sum(4 * v[0].numel() for v in per_chain.values())
+    n = min(C, (DUMP_BYTES - sum(4 * v.numel() for v in shared.values())) // row_bytes)
+    idx = np.arange(C) if n == C else np.sort(np.random.default_rng(0).choice(C, n, replace=False))
+    out = {"chain_index": idx.astype(np.float64)}
+    for k, v in per_chain.items():
+        out[k] = v.index_select(0, torch.from_numpy(idx).to(v.device)).float().cpu().numpy()
+    for k, v in shared.items():
+        out[k] = v.float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_nuts_workload(args, wl, dev, dist, world, rank, local_rank):
     """BASELINE configs[2] (NUTS on the funnel) and configs[3] (NUTS + shared window adaptation).  value = leapfrogs the
     trees actually executed (sum of num_integration_steps over chains, steps and ranks) / max-over-ranks CUDA-event time."""
@@ -377,7 +403,7 @@ def run_nuts_workload(args, wl, dev, dist, world, rank, local_rank):
     if adapt:
         def one_step(t, count):
             (st, params), hist = warm.run(step_keys[t], q0, T, _leapfrog_counter=count)
-            return st, params
+            return st, params, hist
         state = None
     else:
         state = bj.nuts.init(q0.clone(), tgt)
@@ -389,7 +415,7 @@ def run_nuts_workload(args, wl, dev, dist, world, rank, local_rank):
                                                               max_num_doublings=depth, keep_history=False, chain_offset=rank * C)
                 if count is not None:
                     count += n_int.sum()
-                return state, acc
+                return state, acc, n_int
             state, info = kern(step_keys[t], state, tgt, wl["eps"], imm, depth)
             if count is not None:
                 count += info.num_integration_steps.sum()
@@ -416,6 +442,18 @@ def run_nuts_workload(args, wl, dev, dist, world, rank, local_rank):
             clocks = {"sm_mhz": min(c["sm_mhz"] for c in ok), "sm_max_mhz": max(c["sm_max_mhz"] for c in ok),
                       "reasons": sorted(set(r for c in ok for r in c["reasons"])),
                       "per_rank_sm_mhz": [c["sm_mhz"] for c in ok], "samples": sum(c.get("samples", 0) for c in ok)}
+    if args.dump_outputs and rank == 0:
+        if adapt:
+            st, params, hist = out
+            dump_outputs(args.dump_outputs, st._asdict(), {"step_size": [params["step_size"]],
+                                                           "inverse_mass_matrix": params["inverse_mass_matrix"],
+                                                           "step_size_history": hist})
+        elif BLK > 1:   # acceptance rates and tree sizes of the step's BLK transitions, chains first
+            st, acc, n_int = out
+            dump_outputs(args.dump_outputs, {**st._asdict(), "acceptance_rate": acc.T, "num_integration_steps": n_int.T})
+        else:
+            st, info = out
+            dump_outputs(args.dump_outputs, {**st._asdict(), **{k: v for k, v in info._asdict().items() if torch.is_tensor(v)}})
 
     # ---- end to end with HOST buffers: positions in from pinned memory, one step, positions + a per-chain result out -----
     q_host = torch.empty(C, D, dtype=torch.float32).pin_memory()
@@ -544,7 +582,11 @@ def main():
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--e2e-chunks", type=int, default=4, help="chain slices (streams) of the end-to-end leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0's chains) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
@@ -638,6 +680,8 @@ def main():
                 clocks = {"sm_mhz": min(c["sm_mhz"] for c in ok), "sm_max_mhz": max(c["sm_max_mhz"] for c in ok),
                           "reasons": sorted(set(r for c in ok for r in c["reasons"])),
                           "per_rank_sm_mhz": [c["sm_mhz"] for c in ok], "samples": sum(c.get("samples", 0) for c in ok)}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {**state._asdict(), **{k: v for k, v in info._asdict().items() if torch.is_tensor(v)}})
 
     # ---- the vectorised single-step leapfrog kernel: the HBM roofline the north star names -------------
     eng = _engine.get_engine(state.position, tgt)
