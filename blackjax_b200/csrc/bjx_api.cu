@@ -69,6 +69,13 @@ static inline bool use_big_path(bjx_handle_t h) { return h->sc == SC_BIG && !use
     if (e_ != cudaSuccess) return cuda_fail(h, e_, where);        \
   } while (0)
 
+// Dense targets and dense metrics stop at 1024 dims: the tensor-core products accumulate in float32 with truncation at
+// each of their 3K/16 steps, so their error grows linearly in K and passes the 1e-5 per product stated for the path
+// beyond K = 1024 (DESIGN.md section 3).
+constexpr int kDenseMaxDim = 1024;
+constexpr const char* kDenseLimitMsg =
+    "dense targets and dense metrics are built for dim <= 1024 (beyond, the tensor-core products lose float32 accuracy)";
+
 static int validate_target(bjx_handle_t h, const bjx_target_desc& t, int dim) {
   if (t.dim != dim) return fail(h, BJX_E_INVALID, "target.dim != config.dim");
   switch (t.kind) {
@@ -81,6 +88,7 @@ static int validate_target(bjx_handle_t h, const bjx_target_desc& t, int dim) {
     case BJX_TARGET_DENSE_GAUSSIAN:
       if (!t.precision) return fail(h, BJX_E_INVALID, "DENSE_GAUSSIAN target needs precision");
       if (dim > 128 && dim % 4 != 0) return fail(h, BJX_E_UNSUPPORTED, "DENSE_GAUSSIAN target with dim > 128 needs dim % 4 == 0 (tensor-core GEMM path)");
+      if (dim > kDenseMaxDim) return fail(h, BJX_E_UNSUPPORTED, kDenseLimitMsg);
       break;
     case BJX_TARGET_BANANA:
       if (dim != 2) return fail(h, BJX_E_INVALID, "BANANA target needs dim == 2");
@@ -297,6 +305,7 @@ extern "C" int bjx_set_metric(bjx_handle_t h, int32_t kind, const float* imm) {
   } else if (kind == BJX_METRIC_DENSE) {
     if (D > 128 && D % 4 != 0)
       return fail(h, BJX_E_UNSUPPORTED, "dense metric with dim > 128 needs dim % 4 == 0 (tensor-core GEMM path)");
+    if (D > kDenseMaxDim) return fail(h, BJX_E_UNSUPPORTED, kDenseLimitMsg);
     elems = (size_t)D * D;
   } else
     return fail(h, BJX_E_INVALID, "The mass matrix has the wrong number of dimensions: expected 1 or 2");  // metrics.py:724-728

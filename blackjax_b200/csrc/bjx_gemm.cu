@@ -464,7 +464,9 @@ k_gemm_f16x3(const __grid_constant__ CUtensorMap tm_x,   // [K, 2, M]  binary16 
         }
         sts_f4(yo, y);
         if (E.planes) {
-          amax = fmaxf(fmaxf(amax, fmaxf(fabsf(y.x), fabsf(y.y))), fmaxf(fabsf(y.z), fabsf(y.w)));
+          // past the last column the slab holds no Cin (nothing is loaded there): whatever an earlier sub-tile, tile or
+          // kernel left in it must not reach the row maximum
+          if (in_cols) amax = fmaxf(fmaxf(amax, fmaxf(fabsf(y.x), fabsf(y.y))), fmaxf(fabsf(y.z), fabsf(y.w)));
           const float s0 = y.x * sc, s1 = y.y * sc, s2 = y.z * sc, s3 = y.w * sc;
           const uint32_t ha = pack_h2(s0, s1), hb = pack_h2(s2, s3);
           const float2 fa = unpack_h2(ha), fb = unpack_h2(hb);
@@ -481,11 +483,17 @@ k_gemm_f16x3(const __grid_constant__ CUtensorMap tm_x,   // [K, 2, M]  binary16 
       fence_proxy_async();  // generic-proxy writes above -> visible to the TMA engine
       __syncwarp();
       BJX_PROF_END(t3, w_work);
-      if (lane == 0 && in_cols) {
-        if (!(E.debug & 4)) tma_store_2d(&tm_y, yb, n0s, m0s);
-        if (E.planes && !(E.debug & 2)) {
-          tma_store_3d(&tm_p, p1b, n0s, 0, m0s);
-          tma_store_3d(&tm_p, p2b, n0s, 1, m0s);
+      // Invariant: lane 0 commits exactly one bulk group per sub-tile, so the wait_read<NP - 1> above frees the slabs
+      // of sub-tile i - NP.  A sub-tile past the last column stores nothing and commits an empty group (valid in the
+      // PTX ISA); skipping its commit would let the count of groups fall behind the count of sub-tiles, and the wait
+      // would then pass while the last in-column store still reads a slab that is about to be overwritten.
+      if (lane == 0) {
+        if (in_cols) {
+          if (!(E.debug & 4)) tma_store_2d(&tm_y, yb, n0s, m0s);
+          if (E.planes && !(E.debug & 2)) {
+            tma_store_3d(&tm_p, p1b, n0s, 0, m0s);
+            tma_store_3d(&tm_p, p2b, n0s, 1, m0s);
+          }
         }
         tma_store_commit();
       }

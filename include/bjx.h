@@ -15,6 +15,8 @@
  *    driven from host C++ as launches whose row counts stay on the device); the only calls that wait for the
  *    device are bjx_synchronize, bjx_destroy, bjx_nuts_last_stats and -- once per tree doubling -- bjx_nuts_step on the
  *    tensor-core dense path (dense metric / dense target with dim > 128: the products are sized from the row count).
+ *  - Dense metrics and dense Gaussian targets are built for dim <= 1024: beyond, bjx_create / bjx_set_metric return
+ *    BJX_E_UNSUPPORTED (the tensor-core products would miss their 1e-5 per-product accuracy).
  *  - Return value: 0 ok; <0 invalid argument / unsupported configuration (BJX_E_*);
  *    >0 a cudaError_t.  bjx_last_error(handle) returns the text.  No exceptions or
  *    callbacks cross this ABI.  A handle is not thread-safe; distinct handles are independent.
@@ -141,7 +143,7 @@ int bjx_synchronize(bjx_handle_t h);
 
 /* metrics.default_metric / gaussian_euclidean (metrics.py:180-218,221-346): precomputes
  * mass_matrix_sqrt = 1/sqrt(M^-1) (diag) or L^-T with L = chol(M^-1) (dense), metrics.py:701-729.
- * The dense factorisation runs on the host in float64 and synchronises the stream. */
+ * The dense factorisation runs on the host in float64 and synchronises the stream.  Dense: dim <= 1024. */
 int bjx_set_metric(bjx_handle_t h, int32_t metric_kind, const float* inverse_mass_matrix);
 /* metrics.gaussian_euclidean_low_rank(sigma, U, lam) (metrics.py:349-467): M^-1 = diag(sigma) (I + U (Lambda - I) U^T) diag(sigma),
  * sigma [dim] > 0, U [dim, rank] row-major with orthonormal columns, lam [rank] > 0 (device arrays, copied).  Momentum

@@ -449,7 +449,7 @@ def test_dense_velocity_row_scaling_and_non_finite_rows():
 
 
 @pytest.mark.parametrize("D, C, L, pce", [(256, 96, 6, False), (384, 40, 4, True), (256, 8203, 3, False),
-                                          (256, 8200, 2, True),      # >= 8192 chains: two slices on two streams
+                                          (256, 8200, 2, True),      # 33 row tiles, rank 1 of the last one dead
                                           (132, 33, 5, True)])       # padded operand planes
 def test_dense_hmc_transition_matches_oracle(D, C, L, pce):
     tgt, otgt, imm, q = dense_problem(D, C)
